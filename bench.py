@@ -20,7 +20,7 @@ collective touches the data path.
               host cores over a bounded, size-stratified sample of the SAME 512 bins; the warm-up steps sweep the reference's
               concurrency (arena size = bins in flight, sorter threads) and the timed steps use the best setting
 
-Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scale S] [--no-cpu] [--no-secondary]
+Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scale S] [--no-cpu] [--no-secondary] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -417,6 +417,40 @@ def secondary_block(kmc_b200, torch, dev, tstream, args, peak):
     return out
 
 
+DUMP_RECORDS = 1 << 17          # sampled records per pool bin: 8 bins x 2^17 x 4 float64 = 32 MiB of the 64 MiB a dump may take
+
+
+def dump_outputs(out_dir, torch, dev, out_rec_bytes, my, bin_pool_idx, last_rows, d_outs, d_luts):
+    """--dump-outputs: what kmcb200_dev_process_bin returned in the last timed step, as float64 .npy files, so that two builds can be
+    compared output for output (the inputs depend only on the arguments).
+      bin_results.npy   one row per bin of the step in processing order: bin id, pool bin, then the 8 values of d_result
+                        (n_unique, n_cutoff_min, n_cutoff_max, n_total, emitted records, capacity error, format error bits, LSD fallback)
+      lut_<j>.npy       LUT of pool bin j: emitted records per k-mer prefix of LUT_P symbols
+      records_<j>.npy   emitted records of pool bin j, a fixed sample (seed j) of at most DUMP_RECORDS: record index, prefix (from the
+                        LUT), suffix ((K - LUT_P) / 4 bytes, big-endian) and counter (little-endian)
+    Every occurrence of pool bin j in the step writes the same buffers, so the last one's output is pool bin j's output."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    save = lambda name, a: np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+    save("bin_results", [[bid, bin_pool_idx[bid]] + [int(x) for x in r] for bid, r in zip(my, last_rows)])
+    suffix_bytes = (K - LUT_P) // 4
+    for j in sorted({bin_pool_idx[bid] for bid in my}):
+        n = int(next(r[4] for bid, r in zip(my, last_rows) if bin_pool_idx[bid] == j))
+        lut = d_luts[j].cpu().numpy()
+        assert int(lut.sum()) == n, "pool bin %d: LUT holds %d records, the result row %d" % (j, int(lut.sum()), n)
+        idx = np.sort(np.random.default_rng(j).choice(n, size=min(n, DUMP_RECORDS), replace=False))
+        recs = d_outs[j][:n * out_rec_bytes].view(n, out_rec_bytes)[torch.from_numpy(idx).to(dev)].cpu().numpy().astype(np.uint64)
+        suffix = np.zeros(idx.size, dtype=np.uint64)
+        for c in range(suffix_bytes):
+            suffix = (suffix << np.uint64(8)) | recs[:, c]
+        counter = np.zeros(idx.size, dtype=np.uint64)
+        for c in range(out_rec_bytes - 1, suffix_bytes - 1, -1):
+            counter = (counter << np.uint64(8)) | recs[:, c]
+        prefix = np.searchsorted(np.cumsum(lut), idx, side="right")
+        save("lut_%d" % j, lut)
+        save("records_%d" % j, np.stack([idx, prefix, suffix, counter], axis=1))
+
+
 _ORIG_AFFINITY = None
 
 
@@ -473,14 +507,15 @@ def main_ours(args, rank, world, local_rank):
     ctx = kmc_b200.Stage2Context(kmc_b200.Stage2Params(K, True, CUTOFF_MIN, CUTOFF_MAX, COUNTER_MAX, LUT_P), device=local_rank, n_slots=E2E_SLOTS)
     cap = ctx.out_capacity(max(sizes)) + 64
 
-    # ---- value: the pool resident in HBM; every bin of the shard is one kmcb200_dev_process_bin call with its own result row
+    # ---- value: the pool resident in HBM; every bin of the shard is one kmcb200_dev_process_bin call with its own result row.
+    # Each pool bin has its own output and LUT buffers, so after a step they hold what that step returned for every distinct bin.
     d_pool = []
     for b in pool:
         t = torch.zeros(b.size + 64, dtype=torch.uint8, device=dev)
         t[:b.size] = torch.from_numpy(b.data).to(dev)
         d_pool.append(t)
-    d_out = torch.zeros(cap, dtype=torch.uint8, device=dev)
-    d_lut = torch.zeros(ctx.lut_entries, dtype=torch.int64, device=dev)
+    d_outs = [torch.zeros(ctx.out_capacity(b.n_rec) + 64, dtype=torch.uint8, device=dev) for b in pool]
+    d_luts = [torch.zeros(ctx.lut_entries, dtype=torch.int64, device=dev) for _ in pool]
     n_my = max(len(my), 1)
     d_res = torch.zeros((args.steps + 1) * n_my, 8, dtype=torch.int64, device=dev)
     tstream = torch.cuda.Stream(device=dev)          # a real (non-default) stream: the library enqueues on it, torch events time it
@@ -490,7 +525,8 @@ def main_ours(args, rank, world, local_rank):
 
     def run_dev(j, row):
         b = pool[j]
-        ctx.dev_process_bin(0, d_pool[j].data_ptr(), b.size, b.n_rec, b.pack_bytes, d_out.data_ptr(), cap, d_lut.data_ptr(), d_res[row].data_ptr(), stream)
+        ctx.dev_process_bin(0, d_pool[j].data_ptr(), b.size, b.n_rec, b.pack_bytes, d_outs[j].data_ptr(), d_outs[j].numel(), d_luts[j].data_ptr(),
+                            d_res[row].data_ptr(), stream)
 
     def step_dev(s):
         for i, bid in enumerate(my):
@@ -533,6 +569,9 @@ def main_ours(args, rank, world, local_rank):
             r, e = res_all[s * n_my + i], expect[bin_pool_idx[bid]]
             assert np.array_equal(r[:7], e[:7]), "step %d bin %d: %s != %s" % (s, bid, r, e)
             fallbacks += int(r[7])
+    if args.dump_outputs and rank == 0:
+        last = args.steps - 1
+        dump_outputs(args.dump_outputs, torch, dev, ctx.out_rec_bytes, my, bin_pool_idx, res_all[last * n_my:last * n_my + len(my)], d_outs, d_luts)
     t_dev = torch.tensor([dev_ms], dtype=torch.float64, device=dev)
     if dist is not None:
         all_ms = [torch.zeros_like(t_dev) for _ in range(world)]
@@ -637,7 +676,7 @@ def main_ours(args, rank, world, local_rank):
                                    % (rank_ms.index(max(rank_ms)), loads[rank_ms.index(max(rank_ms))], max(rank_ms), max(sizes), 100.0 * max(sizes) / max(loads))},
             "timed_region_s": {"value": dev_ms * 1e-3, "e2e": t_e2e},
         }
-        del d_pool
+        del d_pool, d_outs
         torch.cuda.empty_cache()
         if world == 1 and not args.no_secondary:
             ctx.close()
@@ -664,7 +703,12 @@ def main():
     ap.add_argument("--scale", type=int, default=int(os.environ.get("KMCB200_BENCH_SCALE", "1")), help="divide every bin size by this (development runs)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg (profiling runs)")
     ap.add_argument("--no-secondary", action="store_true", help="skip the secondary workloads (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

@@ -5,8 +5,13 @@
 * ctypes wrappers for the two checkers:
     - `Oracle`     : oracle/_build/libkmc_oracle.so  (our plain-C restatement)
     - `Reference`  : oracle/_ref/libkmc_ref.so       (the unmodified reference classes, when built)
+* what the reference returned for the tests' inputs (tests/golden/reference_results.json, made by
+  tests/golden/make_reference_results.py), so that the comparisons with it run without the reference
 """
 import ctypes as C
+import functools
+import hashlib
+import json
 import os
 import subprocess
 from dataclasses import dataclass, field
@@ -19,6 +24,8 @@ ORACLE_SO = os.path.join(ORACLE_DIR, "_build", "libkmc_oracle.so")
 REF_SO = os.path.join(ORACLE_DIR, "_ref", "libkmc_ref.so")
 REF_B200_SO = os.path.join(ORACLE_DIR, "_ref", "libkmc_ref_b200.so")    # same harness, CKmerBinSorterB200 in place of CKmerBinSorter
 PACK_BYTES = 1 << 16          # bin_part_size, kmc_core/kmc.h:151
+GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
+REFERENCE_RESULTS = os.path.join(GOLDEN_DIR, "reference_results.json")
 
 
 # ----------------------------------------------------------------------------- parameters
@@ -326,6 +333,30 @@ def decode_payload(payload, lut, p: Params):
             res.append((s, c))
             i += 1
     return res
+
+
+# ----------------------------------------------------------------------------- stored reference results
+def sha256(data):
+    return hashlib.sha256(bytes(data)).hexdigest()
+
+
+def result_digest(r):
+    """A bin result (this module's BinResult or kmc_b200's) as reference_results.json stores it: the four counters in
+    the clear, payload and LUT (uint64) by SHA-256."""
+    payload = r.payload if isinstance(r.payload, bytes) else r.payload.tobytes()
+    return {"stats": [int(x) for x in r.stats], "payload_sha256": sha256(payload),
+            "lut_sha256": sha256(np.ascontiguousarray(r.lut, dtype=np.uint64).tobytes())}
+
+
+@functools.lru_cache(maxsize=None)
+def _reference_results():
+    with open(REFERENCE_RESULTS) as f:
+        return json.load(f)
+
+
+def reference_results(group):
+    """What the reference returned for one test module's inputs (a dict keyed by case)."""
+    return _reference_results()[group]
 
 
 # ----------------------------------------------------------------------------- build helpers

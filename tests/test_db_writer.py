@@ -1,21 +1,34 @@
 """The database writer of SURVEY 8f N3 (kmcb200_db_*: pinned staging ring, writer thread, footer) against files written by the REFERENCE:
-a database made by the unmodified reference CLI (oracle/_ref/kmc_ref, one stage-2 sorter so that the bin order is deterministic) is taken
-apart into its bins (payload and LUT of every bin, signature map, header fields) and replayed through the writer; .kmc_pre and .kmc_suf must
-come out byte for byte.  Host-only: runs without a GPU (the staging ring is then plain memory)."""
+a database made by the unmodified reference CLI (one stage-2 sorter so that the bin order is deterministic) is taken apart into its bins
+(payload and LUT of every bin, signature map, header fields) and replayed through the writer; .kmc_pre and .kmc_suf must come out byte
+for byte.  Host-only: runs without a GPU (the staging ring is then plain memory).
+
+The reference's databases are stored in tests/golden/refdb_*.npz, and the SHA-256 of the files the reference's kmc_tools read back
+(with the dump it printed) in tests/golden/reference_results.json ("db_writer"); tests/golden/make_reference_results.py made both."""
 import os
 import struct
 
 import numpy as np
 import pytest
 
-from test_gpu_kmc_files import KMC_REF, write_fastq, count
+from kmc_testlib import GOLDEN_DIR, Params, reference_results, sha256
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+REFDB_CASES = [(31, ("-ci2",)), (28, ("-ci1", "-cs65535")), (55, ("-ci1", "-b"))]
+REFDB_ARGS = ("-sr1", "-n64")          # one stage-2 sorter, 64 bins
+REFDB_STATS = ("#Unique_k-mers", "#k-mers_below_min_threshold", "#k-mers_above_max_threshold", "#Total no. of k-mers")
+STANDALONE_PARAMS = Params(k=31, cutoff_min=2, lut_prefix_len=7)
+STANDALONE_SIG_LEN = 9
 
 
-def parse_db(prefix):
-    pre = open(prefix + ".kmc_pre", "rb").read()
-    suf = open(prefix + ".kmc_suf", "rb").read()
+def refdb_path(k, extra):
+    return os.path.join(GOLDEN_DIR, "refdb_k%d%s.npz" % (k, "".join(extra)))
+
+
+def read_db(prefix):
+    return open(prefix + ".kmc_pre", "rb").read(), open(prefix + ".kmc_suf", "rb").read()
+
+
+def parse_db(pre, suf):
     assert pre[:4] == b"KMCP" and pre[-4:] == b"KMCP" and suf[:4] == b"KMCS" and suf[-4:] == b"KMCS"
     header_offset = struct.unpack("<I", pre[-8:-4])[0]
     h = len(pre) - 8 - header_offset
@@ -38,25 +51,25 @@ def parse_db(prefix):
                 sig_map=sig_map, luts=luts, payloads=payloads, n_recs=n_recs)
 
 
-@pytest.mark.parametrize("k,extra", [(31, ("-ci2",)), (28, ("-ci1", "-cs65535")), (55, ("-ci1", "-b"))])
+@pytest.mark.parametrize("k,extra", REFDB_CASES)
 @pytest.mark.parametrize("raw_lut", [False, True])
 def test_writer_reproduces_reference_files(tmp_path, k, extra, raw_lut):
     import ctypes as C
     import kmc_b200
-    if not os.path.exists(KMC_REF):
-        pytest.skip("oracle/_ref/kmc_ref not built")
     tmp = str(tmp_path)
-    fq = os.path.join(tmp, "reads.fq")
-    write_fastq(fq, 500 + k, 8000)
-    db, stats = count(KMC_REF, tmp, "ref", fq, k, extra + ("-sr1", "-n64"))
-    d = parse_db(db)
-    st = stats["Stats"]
+    z = np.load(refdb_path(k, extra))
+    ref_pre, ref_suf = z["kmc_pre"].tobytes(), z["kmc_suf"].tobytes()
+    d = parse_db(ref_pre, ref_suf)
+    assert d["k"] == k
+    st = dict(zip(REFDB_STATS, z["stats"]))
     out = os.path.join(tmp, "replay")
     w = kmc_b200.DbWriter(out, d["k"], d["counter_size"], d["p"], d["sig_len"], d["cmin"], d["cmax"], d["both"], staging_bytes=1 << 20)   # a small ring: it wraps and blocks
     n_bins = d["luts"].shape[0]
     for b in range(n_bins):
         pay = d["payloads"][b]
-        ptr = w.reserve(len(pay))
+        # every region is 64 KiB larger than its payload (as when a GPU caller reserves the bin's output capacity): the 64 bins pass
+        # through the 1 MiB ring several times
+        ptr = w.reserve(len(pay) + (1 << 16))
         C.memmove(ptr, pay, len(pay))
         lut = d["luts"][b]
         if raw_lut:
@@ -68,8 +81,8 @@ def test_writer_reproduces_reference_files(tmp_path, k, extra, raw_lut):
         w.commit_bin(len(pay), lut, bin_stats, sigs, raw_lut=raw_lut)
     tot = w.close()
     assert tot[0] - tot[1] - tot[2] == d["n_counted"]
-    assert open(out + ".kmc_suf", "rb").read() == open(db + ".kmc_suf", "rb").read()
-    assert open(out + ".kmc_pre", "rb").read() == open(db + ".kmc_pre", "rb").read()
+    assert open(out + ".kmc_suf", "rb").read() == ref_suf
+    assert open(out + ".kmc_pre", "rb").read() == ref_pre
 
 
 def _standalone_bins():
@@ -86,28 +99,40 @@ def _expected_dump(results, p):
     return lines
 
 
-def test_standalone_database_is_readable_by_the_reference_tools(tmp_path, oracle):
-    """Bins -> (oracle results) -> writer -> files; the reference's kmc_tools must read the database back bin after bin."""
+def dump_sha256(results, p):
+    """SHA-256 of what `kmc_tools transform <db> dump` prints for a database of these bin results (one line per record, in file order)."""
+    return sha256("".join(line + "\n" for line in _expected_dump(results, p)).encode())
+
+
+def write_oracle_db(out, results, p, staging_bytes):
+    """A database of bin results through the writer (bin i under signature i, LUTs scanned by the writer)."""
     import ctypes as C
     import kmc_b200
-    from kmc_testlib import Params
-    from test_gpu_kmc_files import KMC_TOOLS, run
-    if not os.path.exists(KMC_TOOLS):
-        pytest.skip("oracle/_ref/kmc_tools not built")
-    p = Params(k=31, cutoff_min=2, lut_prefix_len=7)
-    bins = _standalone_bins()
-    res = [oracle.process_bin(b, p) for b in bins]
-    out = os.path.join(str(tmp_path), "standalone")
-    w = kmc_b200.DbWriter(out, 31, p.counter_bytes, 7, 9, p.cutoff_min, p.cutoff_max, True, staging_bytes=1 << 20)
-    for i, r in enumerate(res):
+    w = kmc_b200.DbWriter(out, p.k, p.counter_bytes, p.lut_prefix_len, STANDALONE_SIG_LEN, p.cutoff_min, p.cutoff_max, p.both_strands,
+                          staging_bytes=staging_bytes)
+    for i, r in enumerate(results):
         ptr = w.reserve(len(r.payload))
         C.memmove(ptr, r.payload, len(r.payload))
         w.commit_bin(len(r.payload), r.lut, r.stats, [i], raw_lut=True)
-    tot = w.close()
+    return w.close()
+
+
+def check_against_reference_tools(out, results, p, case):
+    """The files must be those the reference's kmc_tools read back, and what it printed must be the dump of the bin results."""
+    ref = reference_results("db_writer")[case]
+    pre, suf = read_db(out)
+    assert sha256(pre) == ref["kmc_pre_sha256"] and sha256(suf) == ref["kmc_suf_sha256"]
+    assert dump_sha256(results, p) == ref["dump_sha256"]
+
+
+def test_standalone_database_is_readable_by_the_reference_tools(tmp_path, oracle):
+    """Bins -> (oracle results) -> writer -> files; the reference's kmc_tools must read the database back bin after bin."""
+    p = STANDALONE_PARAMS
+    res = [oracle.process_bin(b, p) for b in _standalone_bins()]
+    out = os.path.join(str(tmp_path), "standalone")
+    tot = write_oracle_db(out, res, p, 1 << 20)
     assert tot == tuple(sum(r.stats[j] for r in res) for j in range(4))
-    txt = os.path.join(str(tmp_path), "dump.txt")
-    run([KMC_TOOLS, "transform", out, "dump", txt])
-    assert open(txt).read().split("\n")[:-1] == _expected_dump(res, p)
+    check_against_reference_tools(out, res, p, "standalone")
 
 
 @pytest.mark.gpu
@@ -115,16 +140,12 @@ def test_gpu_bins_straight_into_the_database(tmp_path, oracle):
     """The standalone stage 2: bins -> kmcb200_submit_bin with the writer's pinned ring as D2H target -> kmcb200_wait_bin_scanned (LUT prefix
     sum on the GPU, base = records so far) -> commit; two bins in flight while the writer thread appends the earlier ones."""
     import kmc_b200
-    from kmc_testlib import Params
-    from test_gpu_kmc_files import KMC_TOOLS, run
-    if not os.path.exists(KMC_TOOLS):
-        pytest.skip("oracle/_ref/kmc_tools not built")
-    p = Params(k=31, cutoff_min=2, lut_prefix_len=7)
+    p = STANDALONE_PARAMS
     bins = _standalone_bins() * 3
     res = [oracle.process_bin(b, p) for b in bins]
     out = os.path.join(str(tmp_path), "gpu_db")
     ctx = kmc_b200.Stage2Context(kmc_b200.Stage2Params(31, True, 2, 10 ** 9, 255, 7), device=0, n_slots=2)
-    w = kmc_b200.DbWriter(out, 31, p.counter_bytes, 7, 9, p.cutoff_min, p.cutoff_max, True, staging_bytes=1 << 18)
+    w = kmc_b200.DbWriter(out, 31, p.counter_bytes, 7, STANDALONE_SIG_LEN, p.cutoff_min, p.cutoff_max, True, staging_bytes=1 << 18)
     luts = [np.zeros(ctx.lut_entries, dtype=np.uint64) for _ in range(2)]
     datas = [np.ascontiguousarray(b.data) for b in bins]
 
@@ -143,6 +164,4 @@ def test_gpu_bins_straight_into_the_database(tmp_path, oracle):
     tot = w.close()
     ctx.close()
     assert tot == tuple(sum(r.stats[j] for r in res) for j in range(4))
-    txt = os.path.join(str(tmp_path), "dump.txt")
-    run([KMC_TOOLS, "transform", out, "dump", txt])
-    assert open(txt).read().split("\n")[:-1] == _expected_dump(res, p)
+    check_against_reference_tools(out, res, p, "standalone_x3")

@@ -4,7 +4,7 @@ import ctypes as C
 import numpy as np
 import pytest
 
-from kmc_testlib import Params, Bin, synth_bin, fast_bin, pack_superkmers, choose_lut_prefix_len, bin_from_reads
+from kmc_testlib import Params, Bin, synth_bin, fast_bin, pack_superkmers, choose_lut_prefix_len, bin_from_reads, reference_results, result_digest
 
 pytestmark = pytest.mark.gpu
 
@@ -354,45 +354,37 @@ def test_leaf_count_crowded_leaf_and_heavy_kmer(oracle):
 
 
 # ----------------------------------------------------------------------------------------------------------------------
-# Round 2: parity at benchmark scale, against the reference itself (oracle/_ref/libkmc_ref.so travels to the GPU box)
-def _reference_or_skip():
-    from kmc_testlib import Reference, reference_available
-    if not reference_available():
-        pytest.skip("oracle/_ref/libkmc_ref.so not built")
-    return Reference()
+# Round 2: parity at benchmark scale, against the reference itself: what the unmodified CKmerBinSorter<SIZE>::ProcessBins + RADULS
+# returned for these bins is stored in tests/golden/reference_results.json ("gpu_parity", made by tests/golden/make_reference_results.py)
+BENCHMARK_SCALE_CASES = [(31, 7), (55, 7)]
 
 
-def _assert_same(r, e, what=""):
-    assert r.stats == tuple(e.stats), what
-    assert np.array_equal(r.lut, e.lut), what
-    assert r.payload.tobytes() == e.payload, what
+def benchmark_scale_bin(k):
+    return fast_bin(2600 + k, k, 1 << 26)
 
 
-@pytest.mark.parametrize("k,p_len", [(31, 7), (55, 7)])
+def second_level_bin():
+    return fast_bin(117, 31, 117_000_000)
+
+
+@pytest.mark.parametrize("k,p_len", BENCHMARK_SCALE_CASES)
 def test_benchmark_scale_bit_exact_vs_reference(k, p_len):
     """One bin of 2^26 k-mers (BASELINE configs[1] / the benchmark's bin size): payload, LUT and statistics byte for byte
     against the unmodified CKmerBinSorter<SIZE>::ProcessBins + RADULS (k=55: against the reference's (k,x)-mer path)."""
-    import os
-    R = _reference_or_skip()
     p = Params(k=k, cutoff_min=2, lut_prefix_len=p_len)
-    b = fast_bin(2600 + k, k, 1 << 26)
     ctx = _ctx(p)
-    r = ctx.process_bin(b)
-    e = R.process_bin(b, p, n_sorters=os.cpu_count() or 8)
-    _assert_same(r, e, "k=%d" % k)
+    r = ctx.process_bin(benchmark_scale_bin(k))
+    assert result_digest(r) == reference_results("gpu_parity")["bin_2^26_k%d_p%d" % (k, p_len)], "k=%d" % k
     assert r.n_total == 1 << 26
     ctx.close()
 
 
 def test_large_second_level_bit_exact_vs_reference():
     """A bin of the target workload's size (1.2e8 k-mers: 9-bit second partition level, 2^17 leaves) against the reference."""
-    import os
-    R = _reference_or_skip()
     p = Params(k=31, cutoff_min=2, lut_prefix_len=7)
-    b = fast_bin(117, 31, 117_000_000)
     ctx = _ctx(p)
-    r = ctx.process_bin(b)
-    _assert_same(r, R.process_bin(b, p, n_sorters=os.cpu_count() or 8))
+    r = ctx.process_bin(second_level_bin())
+    assert result_digest(r) == reference_results("gpu_parity")["bin_117M_k31_p7"]
     ctx.close()
 
 

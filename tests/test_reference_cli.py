@@ -1,12 +1,17 @@
-"""BASELINE configs[0] (CPU plumbing, no GPU): a ~1 MB synthetic FASTQ through the UNMODIFIED reference CLI (oracle/_ref/kmc_ref, built by
-`make -C oracle cli`) at k = 15 (the regular bin pipeline: the small-k direct-count path needs k <= 13, SURVEY section 0.2) and k = 13 (small-k
-path), checked against a brute-force count of the reads (the reference's own test strategy: tests/kmc_CLI/trivial-k-mer-counter).  This pins
-the test infrastructure the whole-file GPU parity tests rest on (the FASTQ writer, the CLI wrappers, kmc_tools dump)."""
+"""BASELINE configs[0] (CPU plumbing, no GPU): a ~1 MB synthetic FASTQ through the UNMODIFIED reference CLI at k = 15 (the regular bin
+pipeline: the small-k direct-count path needs k <= 13, SURVEY section 0.2) and k = 13 (small-k path), checked against a brute-force count
+of the reads (the reference's own test strategy: tests/kmc_CLI/trivial-k-mer-counter).  What the CLI counted (`kmc -ci2 -cs255`, dumped
+by `kmc_tools transform ... dump -s`) is stored in tests/golden/reference_results.json ("reference_cli", made by
+tests/golden/make_reference_results.py).  This pins the FASTQ writer the whole-file GPU parity tests rest on."""
 import os
 
 import pytest
 
-from test_gpu_kmc_files import KMC_REF, KMC_TOOLS, write_fastq, count, dump_sorted
+from kmc_testlib import reference_results, sha256
+from test_gpu_kmc_files import write_fastq
+
+FASTQ = dict(seed=15, n_reads=3400, genome_len=200_000)          # 3400 x 150 bp: ~1 MB of FASTQ
+CLI_ARGS = ("-ci2", "-cs255")
 
 
 def brute_force(fastq, k, both=True):
@@ -26,17 +31,17 @@ def brute_force(fastq, k, both=True):
     return cnt
 
 
+def counts_sha256(counts):
+    """SHA-256 of {k-mer: count} as `kmc_tools transform ... dump -s` prints it: one "kmer<TAB>count" line per k-mer, sorted."""
+    return sha256("".join("%s\t%d\n" % (km, c) for km, c in sorted(counts.items())).encode())
+
+
 @pytest.mark.parametrize("k", [15, 13])
 def test_reference_cli_on_a_small_fastq(tmp_path, k):
-    if not (os.path.exists(KMC_REF) and os.path.exists(KMC_TOOLS)):
-        pytest.skip("oracle/_ref/kmc_ref not built (make -C oracle cli needs /root/reference)")
-    tmp = str(tmp_path)
-    fq = os.path.join(tmp, "reads.fq")
-    write_fastq(fq, 15, 3400, genome_len=200_000)          # 3400 x 150 bp: ~1 MB of FASTQ
+    fq = os.path.join(str(tmp_path), "reads.fq")
+    write_fastq(fq, FASTQ["seed"], FASTQ["n_reads"], genome_len=FASTQ["genome_len"])
     assert 0.9e6 < os.path.getsize(fq) < 1.3e6
-    db, stats = count(KMC_REF, tmp, "ref", fq, k, ("-ci2", "-cs255"))
     exp = {km: min(c, 255) for km, c in brute_force(fq, k).items() if c >= 2}
-    got = dict(l.split() for l in dump_sorted(tmp, db, "ref").splitlines())
-    assert {km: int(c) for km, c in got.items()} == exp
-    st = stats["Stats"]
-    assert int(st["#Unique_counted_k-mers"]) == len(exp)
+    ref = reference_results("reference_cli")["k%d" % k]
+    assert counts_sha256(exp) == ref["dump_sha256"]
+    assert len(exp) == ref["unique_counted_kmers"]
