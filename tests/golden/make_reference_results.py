@@ -4,6 +4,7 @@ without it.  Needs oracle/_ref, built by `make -C oracle ref cli REF=<reference 
   reference_results.json   per test module: bin results (the four counters, SHA-256 of payload and LUT), sorted records (SHA-256),
                            counts of the reference CLI, and databases read back by the reference's kmc_tools (SHA-256 of .kmc_pre,
                            .kmc_suf and of the dump it printed for them)
+                           "benchmark_bins" holds bench.py's own bins, each with a SHA-256 of its input
   refdb_k*.npz             databases written by the reference CLI: .kmc_pre, .kmc_suf and the four counters of its statistics, made
                            from FASTQs small enough to store
 
@@ -13,6 +14,8 @@ import json
 import os
 import sys
 import tempfile
+import time
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 
@@ -21,6 +24,7 @@ TESTS = os.path.dirname(HERE)
 sys.path[:0] = [os.path.dirname(TESTS), TESTS]
 
 from kmc_testlib import Oracle, Params, Reference, REFERENCE_RESULTS, result_digest, sha256  # noqa: E402
+import test_benchmark_bins as tbb  # noqa: E402
 import test_db_writer as dbw  # noqa: E402
 import test_gpu_parity as gp  # noqa: E402
 import test_oracle_vs_reference as ovr  # noqa: E402
@@ -99,11 +103,47 @@ def gpu_parity(R):
     return out
 
 
-def main():
+def benchmark_bins(R):
+    """Every bin bench.py times, one at a time (~1.7e9 k-mers in all).  Every result is also checked against the oracle, so that each
+    stored digest is backed by two independent implementations (8 cores: ~6 min in all, most of it the single-threaded oracle)."""
+    n_sorters = os.cpu_count() or 8
+    oracle = Oracle()
+    out = {}
+    with ThreadPoolExecutor(min(32, n_sorters)) as ex:
+        for case in tbb.ALL_CASES:
+            t0 = time.perf_counter()
+            b = case.make(ex)
+            t1 = time.perf_counter()
+            r = R.process_bin(b, case.params, n_sorters=n_sorters)
+            t2 = time.perf_counter()
+            assert oracle.process_bin(b, case.params).same_as(r), case.key
+            t3 = time.perf_counter()
+            out[case.key] = {"input_sha256": tbb.input_sha256(b), "result": result_digest(r)}
+            print("  %s: generated %.1f s, reference %.1f s, oracle %.1f s" % (case.key, t1 - t0, t2 - t1, t3 - t2), flush=True)
+            del b, r
+    return out
+
+
+GROUPS = {"oracle_vs_reference": lambda R, tmp: oracle_vs_reference(R), "reference_cli": lambda R, tmp: reference_cli(tmp),
+          "db_writer": lambda R, tmp: db_writer(tmp, Oracle()), "gpu_parity": lambda R, tmp: gpu_parity(R),
+          "benchmark_bins": lambda R, tmp: benchmark_bins(R)}
+
+
+def main(groups):
+    """Regenerates the named groups (all of them without arguments) and keeps the others as stored."""
+    unknown = set(groups) - set(GROUPS)
+    if unknown:
+        sys.exit("unknown groups %s; known: %s" % (sorted(unknown), sorted(GROUPS)))
     R = Reference()
+    results = {}
+    if groups and os.path.exists(REFERENCE_RESULTS):
+        with open(REFERENCE_RESULTS) as f:
+            results = json.load(f)
     with tempfile.TemporaryDirectory() as tmp:
-        results = {"oracle_vs_reference": oracle_vs_reference(R), "reference_cli": reference_cli(tmp), "db_writer": db_writer(tmp, Oracle()),
-                   "gpu_parity": gpu_parity(R)}
+        for name in groups or GROUPS:
+            t0 = time.perf_counter()
+            results[name] = GROUPS[name](R, tmp)
+            print(name, "%.0f s" % (time.perf_counter() - t0), flush=True)
     with open(REFERENCE_RESULTS, "w") as f:
         json.dump(results, f, indent=1, sort_keys=True)
         f.write("\n")
@@ -112,4 +152,4 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1:])
